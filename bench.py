@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the THA4 poser hot path on B200 (contract: see the task's bench.py section).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference|torch_cuda] [--workload ...] [--no-extras]
+    python bench.py --gpus N --steps K --warmup W [--impl reference|torch_cuda] [--workload ...] [--no-extras] [--dump-outputs DIR]
 
 A "step" is one poser forward over one batch of synthetic input.  The headline workload is BASELINE.json configs[1]:
 the full five-network poser (mode_07), batch 1 per GPU, the lambda_00 character image, one random pose per step,
@@ -178,14 +178,11 @@ def run_reference(args, rank, world):
         if wl['mode'] == 'mode_07':     # eyebrow cache hot, as in the GPU arm (mode_07.py:56-68)
             dec = tha4_oracle.eyebrow_decomposer(sds['eyebrow_decomposer'], img_b[:, :, 64:192, 192:320])
             kw = dict(cached_decomposer_output=dec)
-        t_start = time.perf_counter()
         for i in range(args.warmup + args.steps):
             t0 = time.perf_counter()
             fn(sds, img_b, poses[(i * b) % 32:(i * b) % 32 + b], **kw)
             if i >= args.warmup:
                 times.append((time.perf_counter() - t0) / b)
-            if times and time.perf_counter() - t_start > 150.0:     # bounded sample: keep the arm within minutes
-                break
     spf = sum(times) / len(times)
     B = wl.get('batch', max(1, wl.get('total', 1) // world))
     line = {
@@ -194,8 +191,8 @@ def run_reference(args, rank, world):
         'scaling': 'strong' if 'total' in wl else 'weak', 'vs_baseline': None, 'dtype': 'f32', 'data': 'synthetic',
         'config': config_for(args.workload, B, world),
         'cpu_baseline': {'value': 1.0 / spf, 'unit': 'frames/s', 'cores': threads, 'kind': 'port',
-                         'sample': '%d timed steps (of %d requested) of %d frame(s) each of the same workload (PyTorch-CPU port of the reference path, '
-                                   '%d of %d host threads)' % (len(times), args.steps, per_step_frames, threads, os.cpu_count() or 1)},
+                         'sample': '%d timed steps of %d frame(s) each of the same workload (PyTorch-CPU port of the reference path, '
+                                   '%d of %d host threads)' % (len(times), per_step_frames, threads, os.cpu_count() or 1)},
         'e2e': {'value': 1.0 / spf, 'unit': 'frames/s', 'h2d_bytes_per_step': 0, 'd2h_bytes_per_step': 0},
         'gpu_launches': 0,
     }
@@ -259,6 +256,26 @@ def _claim_stdout():
         sys.stdout.flush()
         _REAL_STDOUT = os.dup(1)
         os.dup2(2, 1)
+
+
+DUMP_BUDGET_BYTES = 60 << 20          # with the .npy headers, under 64 MB
+
+
+def dump_outputs(out_dir, named):
+    """Writes each (name, tensor) as <out_dir>/<name>.npy in float32.  When the tensors hold more than DUMP_BUDGET_BYTES,
+    each one is written flattened and cut to the same share of its elements, taken at positions drawn from a generator
+    seeded with the tensor's index, so that two runs with the same arguments write element-for-element comparable files."""
+    import numpy
+    os.makedirs(out_dir, exist_ok=True)
+    total = sum(t.numel() for _, t in named)
+    keep = min(1.0, DUMP_BUDGET_BYTES / 4 / max(1, total))
+    for i, (name, t) in enumerate(named):
+        t = t.detach().float()
+        if keep < 1.0:
+            flat = t.reshape(-1)
+            idx = torch.randint(flat.numel(), (max(1, int(flat.numel() * keep)),), generator=torch.Generator().manual_seed(i))
+            t = flat[idx.sort().values.to(flat.device)]
+        numpy.save(os.path.join(out_dir, name + '.npy'), t.cpu().numpy())
 
 
 def emit(line: dict):
@@ -351,8 +368,14 @@ def main():
     ap.add_argument('--no-extras', action='store_true', help='skip the student / pose-sweep / distill / torch-eager sub-objects')
     ap.add_argument('--distill-steps', type=int, default=0, help='0: 1000 at N = 8 (BASELINE configs[4]), 200 otherwise')
     ap.add_argument('--option', action='append', default=[], help='library option name=value (developer A/B runs)')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='after the timed steps, write what the last one returned (the poser '
+                    'outputs, or the student weights of a distill step) as DIR/<name>.npy, float32, at most 64 MB in all')
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'tha4_b200':
+        ap.error('--dump-outputs writes the outputs of the tha4_b200 path only')
 
     rank = int(os.environ.get('RANK', '0'))
     world = int(os.environ.get('WORLD_SIZE', '1'))
@@ -424,13 +447,21 @@ def main():
         l0 = ctx.counter('kernel_launches')
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        for i in range(args.steps):
+        for i in range(args.steps - 1):
             step_resident(args.warmup + i)
+        # only the final step's outputs are kept (for --dump-outputs): holding a step's outputs while the next one runs
+        # would move that step's output buffers, and the library replays a frame as a CUDA graph only when they repeat
+        last = step_resident(args.warmup + args.steps - 1)
         e1.record()
         timer.barrier()
         ms = e0.elapsed_time(e1)
         launches = ctx.counter('kernel_launches') - l0
         clocks = sampler.stop()
+        if args.dump_outputs and rank == 0:      # before any later pass reuses the output buffers
+            named = [('student_weights', distiller.flat)] if distiller is not None else \
+                [('%s_output_%02d' % (wl['mode'], k), t) for k, t in enumerate(last)]
+            dump_outputs(args.dump_outputs, named)
+        del last
 
         # ---------------- end to end through the public API with host buffers ----------------
         img_host = image.unsqueeze(0).contiguous().pin_memory()             # ONE image: a sweep poses it B times

@@ -39,6 +39,7 @@ def pack(outputs_per_pose):
 
 
 def main():
+    torch.set_num_threads(synth.FIXTURE_THREADS)
     os.makedirs(os.path.join(GOLDEN, 'data'), exist_ok=True)
     ref = ref_loader.REFERENCE_ROOT
     for src, dst in (('data/images/lambda_00.png', 'lambda_00.png'),

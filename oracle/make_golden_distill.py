@@ -110,6 +110,7 @@ def _run_iteration(args, key_module, module, batch):
 
 
 def main():
+    torch.set_num_threads(synth.FIXTURE_THREADS)
     torch.manual_seed(0)
     real = {k: torch.load(os.path.join(GOLDEN, 'data', 'lambda_00_%s.pt' % k), map_location='cpu') for k in ('face_morpher', 'body_morpher')}
     body_in, face_in = distill_inputs()

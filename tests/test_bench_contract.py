@@ -26,6 +26,27 @@ def test_reference_arm_prints_one_json_line():
     assert d['e2e'] == {'value': d['value'], 'unit': 'frames/s', 'h2d_bytes_per_step': 0, 'd2h_bytes_per_step': 0}
 
 
+def test_dump_outputs_small_in_full_large_as_a_repeatable_sample(tmp_path, monkeypatch):
+    sys.path.insert(0, ROOT)
+    import numpy
+    import torch
+    import bench
+    small = [('a', torch.arange(12.0).reshape(3, 4)), ('b', torch.ones(5, dtype=torch.float64))]
+    bench.dump_outputs(str(tmp_path / 'small'), small)
+    assert numpy.array_equal(numpy.load(tmp_path / 'small' / 'a.npy'), small[0][1].numpy())
+    assert numpy.load(tmp_path / 'small' / 'b.npy').dtype == numpy.float32
+    monkeypatch.setattr(bench, 'DUMP_BUDGET_BYTES', 4 * 1000)
+    large = [('x', torch.randn(3000)), ('y', torch.randn(2, 500))]
+    for d in ('r1', 'r2'):
+        bench.dump_outputs(str(tmp_path / d), large)
+    sizes = 0
+    for name, t in large:
+        a, b = (numpy.load(tmp_path / d / (name + '.npy')) for d in ('r1', 'r2'))
+        assert numpy.array_equal(a, b) and numpy.isin(a, t.numpy()).all()
+        sizes += a.size
+    assert 900 <= sizes <= 1000
+
+
 def test_round2_default_bench_line_has_the_sub_objects():
     """The round-2 default line (BASELINE configs[1]) carries the other configs as sub-objects and the >= 30x denominator."""
     f = os.path.join(ROOT, 'profiles', 'r02_final_bench_default.json')

@@ -1,11 +1,11 @@
-"""Pins the CPU oracle (oracle/tha4_oracle.py, oracle/gridsample_ref.c) to the reference.
-
- * always: against the committed golden fixtures, which oracle/make_golden.py produced by running the unmodified
-   reference (imported from /root/reference) on seeded weights / the shipped lambda_00 student;
- * when /root/reference is present (build container): against the live reference, full tensors, plus the
-   state_dict key/shape layout of every network.
+"""Pins the CPU oracle (oracle/tha4_oracle.py, oracle/gridsample_ref.c) to the reference, through the committed golden
+fixtures that oracle/make_golden.py, oracle/make_golden_distill.py and oracle/make_golden_pins.py recorded by running the
+unmodified reference on seeded weights / the shipped lambda_00 student: sampled output tensors with full-tensor
+statistics, the state_dict key/shape layout of every network, the pose schema, the image conversions and the
+training schedules.
 """
 import ctypes
+import json
 import os
 
 import numpy
@@ -13,9 +13,20 @@ import pytest
 import torch
 import torch.nn.functional as F
 
-from oracle import image_io, ref_loader, synth, tha4_oracle as O
+from oracle import image_io, synth, tha4_oracle as O
+from oracle.make_golden_pins import display_input, poser_inputs, spread, stats, tile_means
 
 STRIDE, OFFSET = 8, 3
+
+
+@pytest.fixture(autouse=True, scope='module')
+def _fixture_thread_count():
+    """The fixtures were recorded with synth.FIXTURE_THREADS CPU threads; the oracle runs with the same count on every
+    host, because the thread count moves its outputs by ~1e-5."""
+    before = torch.get_num_threads()
+    torch.set_num_threads(synth.FIXTURE_THREADS)
+    yield
+    torch.set_num_threads(before)
 
 
 def _check_against_golden(npz, outputs_per_pose, tol):
@@ -118,25 +129,31 @@ def test_c_oracle_resize_matches_torch(oracle_clib, hi, ho):
     assert (out - ref).abs().max().item() < 3e-7
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason='live reference only exists in the build container')
-def test_oracle_equals_live_reference(teacher_sds, student_sds):
-    mods = ref_loader.build_reference_modules(teacher_sds, student_sds)
-    for name, m in mods['teacher'].items():
-        ref_sd = m.state_dict()
-        assert list(ref_sd.keys()) == list(teacher_sds[name].keys())
-        assert all(ref_sd[k].shape == teacher_sds[name][k].shape for k in ref_sd)
-    for name, m in mods['student'].items():
-        assert list(m.state_dict().keys()) == list(student_sds[name].keys())
-    img = synth.synthetic_image(3, 1)[0]
-    pose = synth.random_poses(1, seed=77)[0]
+def _layout(sd):
+    return '\n'.join('%s %s' % (k, list(v.shape)) for k, v in sd.items())
+
+
+def test_oracle_equals_reference_fixture(golden_dir, teacher_sds, student_sds):
+    """tests/golden/reference_posers.npz holds the reference's own state_dict layouts and its mode_07 / mode_12 / mode_14
+    outputs on these inputs (a spread-out sample of every tensor, the mean of every 32x32 tile, and mean / mean|x| /
+    max|x| of the whole tensor)."""
+    npz = numpy.load(os.path.join(golden_dir, 'reference_posers.npz'))
+    for grp, sds in (('teacher', teacher_sds), ('student', student_sds)):
+        names = sorted(k[len('layout_%s_' % grp):] for k in npz.files if k.startswith('layout_%s_' % grp))
+        assert names == sorted(sds)
+        for name in names:
+            assert _layout(sds[name]) == str(npz['layout_%s_%s' % (grp, name)]), (grp, name)
+    img, pose = poser_inputs()
     with torch.no_grad():
-        for mode, grp, sds in (('mode_07', 'teacher', teacher_sds), ('mode_12', 'teacher', teacher_sds),
-                               ('mode_14', 'student', student_sds)):
-            ref = ref_loader.reference_poser(mode, mods[grp]).get_posing_outputs(img, pose)
+        for mode, sds in (('mode_07', teacher_sds), ('mode_12', teacher_sds), ('mode_14', student_sds)):
             mine = getattr(O, mode + '_outputs')(sds, img, pose)
-            assert len(ref) == len(mine)
-            for a, b in zip(ref, mine):
-                assert a.shape == b.shape and (a - b).abs().max().item() <= 1e-6
+            assert len(mine) == int(npz['%s_count' % mode])
+            for i, b in enumerate(mine):
+                key = '%s_o%02d' % (mode, i)
+                assert list(b.shape) == npz[key + '_shape'].tolist(), key
+                assert numpy.abs(spread(b, 256).numpy() - npz[key]).max() <= 1e-6, key
+                assert numpy.abs(stats(b) - npz[key + '_stats']).max() <= 1e-6, key
+                assert numpy.abs(tile_means(b).astype(numpy.float64) - npz[key + '_tiles']).max() <= 1e-6, key
 
 
 # ------------------------------------------------------------------------------------------ distillation steps (a16-a18)
@@ -184,38 +201,39 @@ def test_distill_oracle_matches_reference_training_iteration_golden(golden_dir, 
         assert (res[net]['after'][::M.GRAD_STRIDE] - after).abs().max().item() <= 2e-7, net
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason='live reference only exists in the build container')
-def test_distill_oracle_equals_live_reference_iteration(lambda00_sds):
-    from oracle import make_golden_distill as M
-    body_in, face_in = M.distill_inputs()
+def test_distill_oracle_equals_reference_iteration_fixture(golden_dir, lambda00_sds):
+    """tests/golden/reference_distill.npz: the gradient and post-Adam parameters of the reference's own training
+    iteration (oracle/make_golden_pins.py), sampled on a different grid than distill_lambda00.npz."""
+    npz = numpy.load(os.path.join(golden_dir, 'reference_distill.npz'))
     res = _distill_oracle_results(lambda00_sds)
-    live = {'body': M.reference_body_step(lambda00_sds['body_morpher'], body_in),
-            'face': M.reference_face_step(lambda00_sds['face_morpher'], face_in)}
     for net in ('body', 'face'):
-        g, gl = res[net]['grad'], live[net]['grad']
-        assert (g - gl).abs().max().item() <= 1e-5 * max(1.0, gl.abs().max().item()), net
-        assert (res[net]['after'] - live[net]['params_after']).abs().max().item() <= 2e-7, net
-        assert abs(sum(res[net]['weighted']) - live[net]['logged']['loss']) <= 5e-6, net
+        g = res[net]['grad']
+        assert g.numel() == int(npz['%s_numel' % net])
+        gl = torch.from_numpy(npz['%s_grad_sub' % net])
+        assert (spread(g, gl.numel()) - gl).abs().max().item() <= 1e-5 * max(1.0, float(npz['%s_grad_absmax' % net])), net
+        after = torch.from_numpy(npz['%s_params_after_sub' % net])
+        assert (spread(res[net]['after'], after.numel()) - after).abs().max().item() <= 2e-7, net
+        assert abs(sum(res[net]['weighted']) - float(npz['%s_logged_loss' % net])) <= 5e-6, net
 
 
 # ------------------------------------------------------------------------------------------ image I/O on either side of the path
-@pytest.mark.skipif(not ref_loader.available(), reason='live reference only exists in the build container')
 def test_image_loader_and_output_conversion_equal_reference(golden_dir):
     """PNG -> poser tensor (full_manual_poser.py:329-339 via extract_pytorch_image_from_filelike) and poser output -> uint8
-    sRGB RGBA (convert_output_image_from_torch_to_numpy, src/tha4/image_util.py:41-58) against the reference's functions."""
-    ref_loader.load()
-    from tha4.shion.base.image_util import extract_pytorch_image_from_filelike
-    from tha4.image_util import convert_output_image_from_torch_to_numpy
+    sRGB RGBA (convert_output_image_from_torch_to_numpy, src/tha4/image_util.py:41-58) against what the reference's
+    functions returned (tests/golden/reference_image_io.npz)."""
     from tha4_b200 import image_util
+    npz = numpy.load(os.path.join(golden_dir, 'reference_image_io.npz'))
     png = os.path.join(golden_dir, 'data', 'lambda_00.png')
-    ref = extract_pytorch_image_from_filelike(png, scale=2.0, offset=-1.0, premultiply_alpha=True, perform_srgb_to_linear=True)
     ours, orc = image_util.load_poser_image(png), image_io.load_rgba_png(png)
-    assert ours.shape == ref.shape == (4, 512, 512)
-    assert (ours - ref).abs().max().item() <= 1e-6 and (orc - ref).abs().max().item() <= 1e-6
+    assert list(ours.shape) == list(orc.shape) == npz['loaded_shape'].tolist() == [4, 512, 512]
+    for t in (ours, orc):
+        assert numpy.abs(spread(t, 8192).numpy() - npz['loaded_sub']).max() <= 1e-6
+        assert numpy.abs(stats(t) - npz['loaded_stats']).max() <= 1e-6
     out = synth.synthetic_image(3, 1)[0]
-    a, b = image_util.poser_output_to_rgba_uint8(out), convert_output_image_from_torch_to_numpy(out)
-    assert a.shape == b.shape == (512, 512, 4) and a.dtype == b.dtype == numpy.uint8
-    assert numpy.abs(a.astype(int) - b.astype(int)).max() <= 1        # uint8 rounding of float32 vs float64 pow
+    a = image_util.poser_output_to_rgba_uint8(out)
+    assert list(a.shape) == npz['output_rgba8_shape'].tolist() == [512, 512, 4] and a.dtype == npz['output_rgba8_sub'].dtype == numpy.uint8
+    a = spread(torch.from_numpy(a), 8192).numpy()
+    assert numpy.abs(a.astype(int) - npz['output_rgba8_sub'].astype(int)).max() <= 1        # uint8 rounding of float32 vs float64 pow
 
 
 def test_image_loader_golden_statistics(golden_dir):
@@ -229,46 +247,44 @@ def test_image_loader_golden_statistics(golden_dir):
 
 
 # ------------------------------------------------------------------------------------------ poser API surface (a1, a2)
-@pytest.mark.skipif(not ref_loader.available(), reason='live reference only exists in the build container')
-def test_pose_schema_and_poser_surface_equal_reference():
+def test_pose_schema_and_poser_surface_equal_reference(golden_dir):
     """Every pose parameter group (name, arity, category, default, range, discreteness -- pose_parameters.py:4-35) and the
-    poser getters the GUIs call (poser.py:132-161) match the reference objects field by field."""
-    ref_loader.load()
-    from tha4.poser.modes.pose_parameters import get_pose_parameters as ref_get
+    poser getters the GUIs call (poser.py:132-161) match the reference objects field by field, as recorded in
+    tests/golden/reference_pins.json."""
     from tha4_b200.poser.modes.pose_parameters import get_pose_parameters as our_get
-    ref, ours = ref_get(), our_get()
-    assert ours.get_parameter_count() == ref.get_parameter_count() == 45
-    rg, og = ref.get_pose_parameter_groups(), ours.get_pose_parameter_groups()
-    assert len(rg) == len(og)
-    for a, b in zip(og, rg):
-        assert a.get_group_name() == b.get_group_name() and a.get_arity() == b.get_arity()
-        assert a.get_parameter_index() == b.get_parameter_index() and a.get_parameter_names() == b.get_parameter_names()
-        assert a.get_category().name == b.get_category().name and a.get_category().value == b.get_category().value
-        assert a.get_default_value() == b.get_default_value() and tuple(a.get_range()) == tuple(b.get_range())
-        assert a.is_discrete() == b.is_discrete()
+    ref = json.load(open(os.path.join(golden_dir, 'reference_pins.json')))['pose']
+    ours = our_get()
+    assert ours.get_parameter_count() == ref['parameter_count'] == 45
+    og = ours.get_pose_parameter_groups()
+    assert len(og) == len(ref['groups'])
+    for a, b in zip(og, ref['groups']):
+        assert a.get_group_name() == b['group_name'] and a.get_arity() == b['arity']
+        assert a.get_parameter_index() == b['parameter_index'] and a.get_parameter_names() == b['parameter_names']
+        assert [a.get_category().name, a.get_category().value] == b['category']
+        assert a.get_default_value() == b['default_value'] and tuple(a.get_range()) == tuple(b['range'])
+        assert a.is_discrete() == b['discrete']
     for i in range(45):
-        assert ours.get_parameter_name(i) == ref.get_parameter_name(i)
-        assert ours.get_parameter_index(ref.get_parameter_name(i)) == i
+        assert ours.get_parameter_name(i) == ref['parameter_names'][i]
+        assert ours.get_parameter_index(ref['parameter_names'][i]) == i
     ssd = synth.student_state_dicts(0)
-    rposer = ref_loader.reference_poser('mode_14', ref_loader.build_reference_modules(None, ssd)['student'])
     from tha4_b200.poser.modes import mode_14
     oposer = mode_14.create_poser(torch.device('cuda:0'), state_dicts=ssd)          # construction needs no GPU (lazy modules)
-    assert oposer.get_image_size() == rposer.get_image_size() and oposer.get_output_length() == rposer.get_output_length()
-    assert oposer.get_num_parameters() == rposer.get_num_parameters() and oposer.get_dtype() == rposer.get_dtype()
+    rposer = ref['mode_14_poser']
+    assert oposer.get_image_size() == rposer['image_size'] and oposer.get_output_length() == rposer['output_length']
+    assert oposer.get_num_parameters() == rposer['num_parameters'] and str(oposer.get_dtype()) == rposer['dtype']
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason='reference checkout not present')
-def test_display_conversion_pinned_to_reference_functions():
+def test_display_conversion_pinned_to_reference_functions(golden_dir):
     """oracle/image_io.frame_to_srgb8 restates the puppeteers' post-processing (a wx app that cannot be imported here);
-    its building blocks are the reference's own convert_linear_to_srgb / torch_linear_to_srgb."""
-    ref_loader.load()
-    from tha4.image_util import convert_linear_to_srgb
-    from oracle import image_io
-    x = synth.synthetic_image(3, 1)[0] * 1.05
+    its building blocks are the reference's own convert_linear_to_srgb / torch_linear_to_srgb, whose results on this
+    input are recorded in tests/golden/reference_image_io.npz."""
+    npz = numpy.load(os.path.join(golden_dir, 'reference_image_io.npz'))
+    x = display_input()
     o = torch.clip((x + 1.0) / 2.0, 0.0, 1.0)
-    assert torch.equal(convert_linear_to_srgb(o), torch.cat([image_io.linear_to_srgb_torch(o[0:3]), o[3:4]], dim=0))
+    srgb = torch.cat([image_io.linear_to_srgb_torch(o[0:3]), o[3:4]], dim=0)
+    assert numpy.array_equal(spread(srgb, 8192).numpy(), npz['display_srgb_sub'])
+    assert numpy.abs(stats(srgb) - npz['display_srgb_stats']).max() <= 1e-9
     plain = image_io.frame_to_srgb8(x, 0)
-    want = (255.0 * convert_linear_to_srgb(o)).permute(1, 2, 0).byte()
-    assert torch.equal(plain, want)
+    assert numpy.array_equal(spread(plain, 8192).numpy(), npz['display_srgb8_sub'])
     white = image_io.frame_to_srgb8(x, 4)
     assert (white[:, :, 3] == 255).all()
